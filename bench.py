@@ -66,7 +66,15 @@ def parse_args(argv=None):
                         "pp: layer-range pipeline, one micro-batch group per stage (the reference's sharding).  "
                         "ep: every rank runs all layers on its own --batch sequences (data-parallel attention) and the routed "
                         "experts of every MoE layer are sharded over the ranks with the fused all-to-all (BASELINE config 5)")
-    return p.parse_args(argv)
+    p.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                   help="after the timed decode steps, write what the last step returned as DIR/<name>.npy: the sampled token ids "
+                        "(float64) and the fp32 logits of every sequence, at most 64 MB in all (logits that do not fit keep a fixed, "
+                        "seeded subset of vocabulary columns).  Inputs are seeded, so two builds run with the same arguments can be "
+                        "compared output for output")
+    args = p.parse_args(argv)
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs records the outputs of --impl ours")
+    return args
 
 
 def reference_arm(args):
@@ -249,6 +257,39 @@ def merge_results(pp, ep):
     return dict(pp, also_measured={"expert parallel (config 5)": brief(ep)})
 
 
+DUMP_BYTES = 64_000_000
+
+
+def decode_outputs(loop, prefix=""):
+    """What the last decode step of ``loop`` handed back on this rank, one row per sequence of every group: the sampled token
+    ids (held by the first stage, where they feed the next step) and the logits (computed by the last stage)."""
+    import torch
+
+    out = {}
+    if loop.first:
+        toks = [loop.p2p.token_inbox(g, loop.B) if loop.transport == "fused" else loop.groups[g].tokens for g in range(loop.G)]
+        out[prefix + "tokens"] = torch.stack(toks)
+    if loop.last:
+        out[prefix + "logits"] = torch.stack(loop._outs)
+    return out
+
+
+def dump_outputs(out_dir, arrays, world):
+    """Write ``name -> tensor`` as ``out_dir/<name>.npy``: token ids as float64 (exact), the rest as float32.  A run writes at
+    most ``world + 1`` logits arrays (pp: the last stage's; ep: one per rank), so each gets that share of ``DUMP_BYTES``
+    (less 1 MB for the token ids); a larger one keeps a fixed, seeded subset of its last-axis columns."""
+    import numpy as np
+
+    budget = (DUMP_BYTES - 1_000_000) // (world + 1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy().astype(np.float32 if t.is_floating_point() else np.float64)
+        if a.nbytes > budget:
+            keep = budget // (a.nbytes // a.shape[-1])
+            a = a[..., np.sort(np.random.default_rng(0).choice(a.shape[-1], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_pp(args, world, rank, local, dev):
     """Layer-range pipeline: one stage per GPU, one micro-batch group per stage in flight, fused P2P hand-off."""
     import torch
@@ -391,6 +432,8 @@ def run_pp(args, world, rank, local, dev):
         dist.barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
     loop.drain()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, decode_outputs(loop), world)
     p2p_err = bool(loop.p2p.error()) if loop.p2p is not None else False
     launches = (loop.launches_per_step * G * args.steps) if loop.use_graphs else ((C.launch_count() - n_launch0) if C else 0)
     ms_per_step = ms / args.steps
@@ -526,6 +569,8 @@ def run_ep(args, world, rank, local, dev):
         torch.cuda.synchronize()
     dist.barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, decode_outputs(loop, prefix=f"ep_rank{rank}_"), world)
     launches = (loop.launches_per_step * args.steps) if loop.use_graphs else (C.launch_count() - n_launch0)
     ms_per_step = ms / args.steps
     tok_s = world * B * 1000.0 / ms_per_step

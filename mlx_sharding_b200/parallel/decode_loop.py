@@ -220,7 +220,7 @@ class DecodeLoop:
                 self.groups[g].graph.replay()
                 out = self._outs[g]
             else:
-                out = self._body(g)
+                out = self._outs[g] = self._body(g)
             self._nccl_post(g, out)
             self._steps_done[g] += 1
 

@@ -92,14 +92,20 @@ def test_console_script_targets_exist():
     assert a.llm_shard_addresses == "h:1,h:2" and a.start_layer == 0 and a.end_layer == 14 and a.cache_limit_gb == 4
 
 
-def test_bench_result_merge_and_reference_arm(capsys):
-    """bench.py host-side contract pieces that need no GPU: the pp/ep result merge and the reference arm's JSON line."""
+def _bench_module():
     import importlib.util
-    import json
 
     spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(REPO, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_result_merge_and_reference_arm(capsys):
+    """bench.py host-side contract pieces that need no GPU: the pp/ep result merge and the reference arm's JSON line."""
+    import json
+
+    bench = _bench_module()
     pp = dict(value=60.0, ms_per_step=8.0, config={"parallelism": "pp8"}, ttft_p50_ms=8.0, ttft_microbatch_ms=60.0, e2e=None,
               gpu_launches=1, clocks={}, metric="m")
     ep = dict(pp, value=99.0, config={"parallelism": "ep8+dp8"})
@@ -115,3 +121,44 @@ def test_bench_result_merge_and_reference_arm(capsys):
     assert line["impl"] == "reference" and "unavailable" in line
     a = bench.parse_args([])
     assert a.gpus == 1 and a.warmup >= 3 and a.parallelism == "auto"
+
+
+def test_bench_dump_outputs(tmp_path):
+    """``bench.py --dump-outputs``: the last decode step's token ids (float64) and fp32 logits as .npy; logits over the size
+    budget keep a seeded column subset that is the same from run to run."""
+    import numpy as np
+
+    from helpers import TINY_DSV2
+    from mlx_sharding_b200.config import ModelConfig
+    from mlx_sharding_b200.ops.meta import BatchMeta
+    from mlx_sharding_b200.parallel.decode_loop import DecodeLoop
+    from mlx_sharding_b200.parallel.pipeline import StageExecutor
+    from mlx_sharding_b200.utils.loader import random_model
+
+    bench = _bench_module()
+    assert bench.parse_args(["--dump-outputs", str(tmp_path)]).dump_outputs == str(tmp_path)
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--dump-outputs", str(tmp_path), "--impl", "baseline"])
+
+    cfg = ModelConfig.from_dict(TINY_DSV2)
+    B, S, PS, steps = 3, 6, 4, 3
+    pps = (S + steps + 2 + PS - 1) // PS
+    stage = StageExecutor(random_model(TINY_DSV2, dtype=torch.float32), B * pps + 1, PS)
+    prompts = torch.randint(3, cfg.vocab_size - 1, (B, S), generator=torch.Generator().manual_seed(3))
+    bts = [[1 + b * pps + i for i in range(pps)] for b in range(B)]
+    first = stage.forward(prompts.reshape(-1), BatchMeta.build([S] * B, [0] * B, bts, PS)).argmax(-1)
+    loop = DecodeLoop(stage, 1, B, pps, use_graphs=False)
+    loop.groups[0].load(torch.full((B,), S, dtype=torch.int32), torch.tensor(bts, dtype=torch.int32), first, S + steps + 2)
+    loop.capture()
+    for _ in range(steps):
+        loop.step_all()
+    bench.dump_outputs(str(tmp_path / "full"), bench.decode_outputs(loop), 1)
+    toks, logits = np.load(tmp_path / "full" / "tokens.npy"), np.load(tmp_path / "full" / "logits.npy")
+    assert toks.dtype == np.float64 and toks.shape == (1, B) and logits.dtype == np.float32 and logits.shape == (1, B, cfg.vocab_size)
+    assert (toks[0] == logits[0].argmax(-1)).all()           # greedy: the step's sampled ids are its logits' argmax
+
+    bench.DUMP_BYTES = 1_000_000 + 2 * B * 100 * 4           # room for 100 of the 320 vocabulary columns
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"logits": torch.from_numpy(logits)}, 1)
+    a, b = np.load(tmp_path / "a" / "logits.npy"), np.load(tmp_path / "b" / "logits.npy")
+    assert a.shape == (1, B, 100) and (a == b).all() and set(a[0, 0].tolist()) <= set(logits[0, 0].tolist())

@@ -31,7 +31,9 @@ def servers(tmp_path_factory):
     path = write_synthetic_checkpoint(str(d / "tiny"), TINY_LLAMA, dtype=torch.float32)
     cwd = os.getcwd()
     os.chdir(d)
-    args = openai_api.build_arg_parser().parse_args(["--model", path, "--port", "0", "--kv-pages", "128", "--page-size", "16"])
+    # the tiny model's head dim (16) has no sm_100a attention kernel: keep it on the CPU path on a machine with a GPU too
+    args = openai_api.build_arg_parser().parse_args(["--model", path, "--port", "0", "--kv-pages", "128", "--page-size", "16",
+                                                     "--device", "cpu"])
     args.static_dir = os.path.join(os.path.dirname(openai_api.__file__), "static")
     provider = openai_api.ModelProvider(args, [])
     httpd = openai_api.make_server("127.0.0.1", 0, provider, args.static_dir)          # in-process server: the oracle
