@@ -49,7 +49,7 @@ def main():
              for _ in range(L)]
     g2 = torch.Generator(device="cuda").manual_seed(100 + rank)
     x0 = torch.randn(T, H, device="cuda", generator=g2).to(torch.bfloat16)
-    bufs = EPBuffers(H, max(T, 64), k)
+    bufs = EPBuffers(H, max(T, 64), k, experts_per_rank=E // world)
     eps = [ExpertParallelMoE(bufs, Wg, Wu, Wd, E) for (Wg, Wu, Wd, _) in banks]
 
     def run_local(x):
@@ -85,28 +85,29 @@ def main():
         return max_over_ranks(e0.elapsed_time(e1)) * 1e3 / (args.iters * L), out
 
     if args.breakdown:
-        # eager, event-timed phases of one EP block on this rank (launch gaps included; flag waits show up in regroup / wait)
+        # eager, event-timed phases of one EP block on this rank, the calls of ExpertParallelMoE.forward (launch gaps included; the
+        # arrival wait shows up in gate_up, the return wait in combine)
         ep, (_, _, _, gate) = eps[0], banks[0]
         b, C, W = bufs, bufs.C, world
-        st = b.state
-        names = ["route", "dispatch", "regroup(wait+bucket)", "gate_up", "down(+fused return)", "combine(+wait)"]
+        names = ["route", "dispatch", "gate_up(+arrival wait)", "down(+return)", "combine(+wait)"]
         acc = [0.0] * len(names)
         n_it = 20
         exp_rows = T * k
+        stride = b.stride(T)
+        rows, row_dst = b.recv_views(stride)
+        mr = min(W * T, stride)
+        arrive = (stride, b.base + b.off_recv_count, b.seq, b.error_ptr, W)
         for it in range(n_it + 3):
             evs = [torch.cuda.Event(enable_timing=True) for _ in range(len(names) + 1)]
             dist.barrier()
             evs[0].record()
             idx, w = b200.moe_route(x0, gate, k); evs[1].record()
-            C.ep_dispatch(x0, idx, ep.E_local, b.rank, b.cap, b.t_recv_x, b.t_recv_meta, b.t_recv_count, st[W + 4:W + 5], st[:W], st[W:W + 1],
-                          st[W + 3:W + 4]); evs[2].record()
-            offs, total, x_perm, row_dst = C.ep_regroup(b.base + b.off_recv_count, st[W + 2:W + 3].data_ptr(), st[-1:].data_ptr(),
-                                                                  b.base + b.off_recv_meta, b.base + b.off_recv_x, W,
-                                                                  b.cap, ep.E_local, b.H, b.dev, W * T * k, b.t_ret_y); evs[3].record()
-            mr = min(W * T, x_perm.shape[0])
-            h = C.grouped_linear(x_perm, ep.wg, ep.wu, offs, mr, ep.act, False, None, None, None, exp_rows); evs[4].record()
-            C.grouped_linear(h, ep.wd, None, offs, mr, 0, True, row_dst, b.ret_flags_dev, st[W + 1:W + 2], exp_rows); evs[5].record()
-            C.ep_combine(b.base + b.off_flags + 128, st[W + 3:W + 4], st[-1:].data_ptr(), b.ret_y, w, x0, None); evs[6].record()
+            C.ep_dispatch_scatter(x0, idx, ep.E_local, b.rank, stride, b.t_recv_x, b.t_recv_meta, b.t_cnt, b.t_recv_count, b.t_my_ret,
+                                  b.seq, b.done, b.ret_expected); evs[2].record()
+            h = C.grouped_linear(rows, ep.wg, ep.wu, b.cnt, mr, ep.act, False, None, None, None, exp_rows, *arrive, True); evs[3].record()
+            C.grouped_linear(h, ep.wd, None, b.cnt, mr, 0, True, row_dst, b.ret_flags_dev, b.tiles, exp_rows, *arrive, False)
+            evs[4].record()
+            C.ep_combine(b.base + b.off_flags + 128, b.ret_expected, b.error_ptr, b.ret_y, w, x0, None); evs[5].record()
             torch.cuda.synchronize()
             if it >= 3:
                 for i in range(len(names)):

@@ -255,8 +255,6 @@ class StageModel:
                 li += 1
             if sp.runs_mlp(i):
                 h = self.mlp_block(i, h, meta)
-        if hasattr(self.ops, "join_aside"):
-            self.ops.join_aside()       # side-stream L2 prefetches (ops/b200.py::prefetch_aside) rejoin here: one join per forward
         if self.spec.is_last:
             return self.head(h, meta, all_logits)
         return h

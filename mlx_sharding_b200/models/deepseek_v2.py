@@ -21,6 +21,7 @@ from typing import Dict
 import torch
 
 from ..ops import BatchMeta, LinearWeight
+from ..parallel.ep import ExpertParallelMoE
 from .base import StageModel, deepseek_rope_spec
 
 _EXPERT_RE = re.compile(r"^(model\.layers\.\d+\.mlp)\.experts\.(\d+)\.(gate_proj|up_proj|down_proj)\.(weight|scales|biases)$")
@@ -163,14 +164,6 @@ class DeepseekV2Stage(StageModel):
             # decode step on the absorbed weights: one GEMM -> [q_abs | q_pe] x 16 heads, c_kv, k_pe; fused prologue (latent norm,
             # both ropes, cache append); tcgen05 multi-query attention over the cached latent; folded output projection
             qkv = O.linear(normed, w["qkv_abs"])
-            if self.backend_name == "b200" and "router" in w and w.get("e_gate") is not None and not w["e_gate"].is_quantized \
-                    and not O.fp8_experts_enabled(w["e_gate"]):
-                nb = O.l2_prefetch_bytes()
-                if nb > 0 and T <= 128:
-                    # forked AFTER the q/kv projection (the chain's bandwidth-hungry kernel): HBM mostly idles from here to the
-                    # expert GEMMs.  Pull the first experts of this layer's gate / up banks into L2 on the side stream (the grouped
-                    # GEMM walks the experts in order, so these are the tiles of its first waves)
-                    O.prefetch_aside([O._dense(w["e_gate"]), O._dense(w["e_up"])], nb)
             qa = qkv[:, : nh * (lr + rd)].unflatten(1, (nh, lr + rd))
             O.mla_absorbed_prologue(qa, qkv[:, nh * (lr + rd): nh * (lr + rd) + lr], qkv[:, nh * (lr + rd) + lr:], w["kv_a_ln"],
                                     c.rms_norm_eps, kpool, meta, self.rope)
@@ -357,82 +350,71 @@ class DeepseekV2Stage(StageModel):
     def mlp_block(self, i, h, meta: BatchMeta):
         O, c, w = self.ops, self.cfg, self.layer_weights[i]
         T = h.shape[0]
-        ep = getattr(self, "ep_layers", None)
-        if "router" in w and "s_gate" not in w and hasattr(O, "moe_block") and not (ep is not None and i in ep):
-            # CUDA backend, whole bank local, shared experts riding in the bank: the block is router -> grouped gate-up -> grouped
-            # down -> combine, with BOTH RMSNorms around it folded in — the pre-MoE norm into the router kernel and the next layer's
-            # input norm into the combine (decode batches; ops/b200.py::moe_block falls back to separate norm kernels otherwise)
-            extra = dict(extra=w["n_fused_shared"]) if "n_fused_shared" in w else {}
-            fk = self._final_kwargs(i, T, "mlp")
-            nxt = self.layer_weights.get(i + 1) if not fk else None
-            nn = dict(next_norm=(nxt["in_ln"], c.rms_norm_eps)) if (nxt is not None and "in_ln" in nxt and self.spec.runs_attn(i + 1)) else {}
-            res = O.moe_block(h, w["router"], dict(top_k=c.num_experts_per_tok, method=c.topk_method, n_group=c.n_group or 1,
-                                                   topk_group=c.topk_group or 1, scaling=c.routed_scaling_factor,
-                                                   norm_topk=c.norm_topk_prob),
-                              w["e_gate"], w["e_up"], w["e_down"], "silu", residual=h, pre_norm=(w["post_ln"], c.rms_norm_eps),
-                              **extra, **nn, **fk)
-            if nn:
-                self._prenormed = res
-                return res[0]
-            return res
-        if ("router" in w and ep is not None and i in ep and hasattr(ep[i], "route_forward") and getattr(ep[i].b, "v2", False)
-                and 1 <= T <= 1024 and os.environ.get("MLXB200_EP_FUSED_ROUTE", "1") != "0"):
+        if "router" not in w:
+            normed = O.rmsnorm(h, w["post_ln"], c.rms_norm_eps)
+            return O.linear(O.gated_up(normed, w["gate"], w["up"], "silu"), w["down"], residual=h,
+                            **self._final_kwargs(i, T, "mlp"))
+        route_kw = dict(top_k=c.num_experts_per_tok, method=c.topk_method, n_group=c.n_group or 1, topk_group=c.topk_group or 1,
+                        scaling=c.routed_scaling_factor, norm_topk=c.norm_topk_prob)
+        ep = (getattr(self, "ep_layers", None) or {}).get(i)
+        cuda = self.backend_name == "b200"
+        nxt = self.layer_weights.get(i + 1)
+        next_norm = (nxt["in_ln"], c.rms_norm_eps) if (nxt is not None and "in_ln" in nxt and self.spec.runs_attn(i + 1)) else None
+        if isinstance(ep, ExpertParallelMoE) and 1 <= T <= 1024:
             # expert-parallel block as four kernels (parallel/ep.py::route_forward): [pre-MoE norm + router + dispatch] -> grouped
             # gate/up -> grouped down (+ return) -> [combine + next layer's input norm]; the shared experts fork onto the side
             # stream right behind the router (they consume the normalised rows it stores)
             def shared_branch(normed):
                 if "s_gate" not in w:
                     return h, None
-                if self.overlap_shared_experts and hasattr(O, "run_aside"):
+                if self.overlap_shared_experts:
                     hs = torch.empty_like(h)
                     return hs, O.run_aside(lambda: O.linear(O.gated_up(normed, w["s_gate"], w["s_up"], "silu"), w["s_down"], residual=h, out=hs))
                 return O.linear(O.gated_up(normed, w["s_gate"], w["s_up"], "silu"), w["s_down"], residual=h), None
 
-            nxt = self.layer_weights.get(i + 1)
-            nn = (nxt["in_ln"], c.rms_norm_eps) if (nxt is not None and "in_ln" in nxt and self.spec.runs_attn(i + 1)) else None
-            res = ep[i].route_forward(h, w["router"], dict(top_k=c.num_experts_per_tok, method=c.topk_method, n_group=c.n_group or 1,
-                                                           topk_group=c.topk_group or 1, scaling=c.routed_scaling_factor,
-                                                           norm_topk=c.norm_topk_prob),
-                                      (w["post_ln"], c.rms_norm_eps), shared_branch, next_norm=nn)
-            if nn is not None:
+            res = ep.route_forward(h, w["router"], route_kw, (w["post_ln"], c.rms_norm_eps), shared_branch, next_norm=next_norm)
+            if next_norm is not None:
+                self._prenormed = res
+                return res[0]
+            return res
+        extra = dict(extra=w["n_fused_shared"]) if "n_fused_shared" in w else {}
+        if ep is None and cuda and "s_gate" not in w:
+            # CUDA backend, whole bank local, shared experts riding in the bank: the block is router -> grouped gate-up -> grouped
+            # down -> combine, with BOTH RMSNorms around it folded in — the pre-MoE norm into the router kernel and the next layer's
+            # input norm into the combine (decode batches; ops/b200.py::moe_block runs separate norm kernels for larger ones)
+            fk = self._final_kwargs(i, T, "mlp")
+            nn = dict(next_norm=next_norm) if (next_norm is not None and not fk) else {}
+            res = O.moe_block(h, w["router"], route_kw, w["e_gate"], w["e_up"], w["e_down"], "silu", residual=h,
+                              pre_norm=(w["post_ln"], c.rms_norm_eps), **extra, **nn, **fk)
+            if nn:
                 self._prenormed = res
                 return res[0]
             return res
         normed = O.rmsnorm(h, w["post_ln"], c.rms_norm_eps)
-        if "router" in w:
-            join = None
-            if "s_gate" in w:
-                # shared experts: h += down(silu(gate x) * up x).  Independent of the routed path until the final combine, so the
-                # CUDA backend runs the two GEMMs on a side stream (a parallel branch of the decode graph) while the main
-                # stream does router -> permutation / expert all-to-all -> expert GEMMs; the combine joins them.
-                if self.overlap_shared_experts and hasattr(O, "run_aside") and self.backend_name == "b200":
-                    hs, h_in = torch.empty_like(h), h   # result buffer allocated before the fork
-                    join = O.run_aside(lambda: O.linear(O.gated_up(normed, w["s_gate"], w["s_up"], "silu"), w["s_down"],
-                                                        residual=h_in, out=hs))
-                    h = hs
-                else:
-                    h = O.linear(O.gated_up(normed, w["s_gate"], w["s_up"], "silu"), w["s_down"], residual=h)
-            extra = dict(extra=w["n_fused_shared"]) if "n_fused_shared" in w else {}
-            ep = getattr(self, "ep_layers", None)
-            if hasattr(O, "moe_block") and join is None and not (ep is not None and i in ep):
-                # CUDA backend, whole bank local: router + experts as one op (scatter path for decode batches, ops/b200.py)
-                return O.moe_block(normed, w["router"], dict(top_k=c.num_experts_per_tok, method=c.topk_method, n_group=c.n_group or 1,
-                                                             topk_group=c.topk_group or 1, scaling=c.routed_scaling_factor,
-                                                             norm_topk=c.norm_topk_prob),
-                                   w["e_gate"], w["e_up"], w["e_down"], "silu", residual=h, **extra, **self._final_kwargs(i, T, "mlp"))
-            idx, wts = O.moe_route(normed, w["router"], c.num_experts_per_tok, c.topk_method,
-                                   c.n_group or 1, c.topk_group or 1, c.routed_scaling_factor,
-                                   c.norm_topk_prob, **extra)
-            ep = getattr(self, "ep_layers", None)
-            if ep is not None and i in ep:
-                # expert-parallel mode (parallel/ep.py): routed experts are sharded over the ranks of the NVSwitch
-                # domain, tokens travel through the fused dispatch / return kernels
-                return ep[i].forward(normed, idx, wts, residual=h, join=join)
-            kw = dict(join=join) if join is not None else {}
-            return O.moe_experts(normed, idx, wts, w["e_gate"], w["e_up"], w["e_down"], "silu", residual=h,
-                                 **kw, **self._final_kwargs(i, T, "mlp"))
-        return O.linear(O.gated_up(normed, w["gate"], w["up"], "silu"), w["down"], residual=h,
-                        **self._final_kwargs(i, T, "mlp"))
+        join = None
+        if "s_gate" in w:
+            # shared experts: h += down(silu(gate x) * up x).  Independent of the routed path until the final combine, so the
+            # CUDA backend runs the two GEMMs on a side stream (a parallel branch of the decode graph) while the main
+            # stream does router -> permutation / expert all-to-all -> expert GEMMs; the combine joins them.
+            if self.overlap_shared_experts and cuda:
+                hs, h_in = torch.empty_like(h), h   # result buffer allocated before the fork
+                join = O.run_aside(lambda: O.linear(O.gated_up(normed, w["s_gate"], w["s_up"], "silu"), w["s_down"],
+                                                    residual=h_in, out=hs))
+                h = hs
+            else:
+                h = O.linear(O.gated_up(normed, w["s_gate"], w["s_up"], "silu"), w["s_down"], residual=h)
+        if ep is None and cuda and join is None:
+            # CUDA backend, whole bank local: router + experts as one op (scatter path for decode batches, ops/b200.py)
+            return O.moe_block(normed, w["router"], route_kw, w["e_gate"], w["e_up"], w["e_down"], "silu", residual=h, **extra,
+                               **self._final_kwargs(i, T, "mlp"))
+        idx, wts = O.moe_route(normed, w["router"], **route_kw, **extra)
+        if ep is not None:
+            # expert-parallel mode (parallel/ep.py): routed experts are sharded over the ranks of the NVSwitch domain, tokens
+            # travel through the fused dispatch / return kernels (all-to-all collectives on the reference backend)
+            return ep.forward(normed, idx, wts, residual=h, join=join)
+        kw = dict(join=join) if join is not None else {}
+        return O.moe_experts(normed, idx, wts, w["e_gate"], w["e_up"], w["e_down"], "silu", residual=h, **kw,
+                             **self._final_kwargs(i, T, "mlp"))
 
 
 Model = DeepseekV2Stage

@@ -188,11 +188,16 @@ def paged_attention(q, kpool, vpool, meta: BatchMeta, scale: float, softcap: flo
                                float(softcap or 0.0), int(meta.max_ctx_len))
 
 
+def route_groups(method: str, n_group: int, topk_group: int) -> Tuple[int, int]:
+    """``(n_group, topk_group)`` the router kernels run with: group-limited top-k only for ``method == "group_limited_greedy"``,
+    one group of all experts for every other method."""
+    return (int(n_group), int(topk_group)) if method == "group_limited_greedy" else (1, 1)
+
+
 def moe_route(x, gate_w, top_k: int, method: str = "greedy", n_group: int = 1, topk_group: int = 1,
               scaling: float = 1.0, norm_topk: bool = False, extra: int = 0):
     """``extra``: always-on experts appended to the routed bank (ids E .. E+extra-1, weight 1.0) — see ``fuse_shared_experts``."""
-    if method != "group_limited_greedy":
-        n_group, topk_group = 1, 1
+    n_group, topk_group = route_groups(method, n_group, topk_group)
     idx, w = C().moe_route(x, _bf16(gate_w), int(top_k), int(n_group), int(topk_group), float(scaling), bool(norm_topk), int(extra))
     return idx, w
 
@@ -231,47 +236,6 @@ def run_aside(fn) -> _Join:
     return _Join(done)
 
 
-_aside_last = {}
-
-
-def prefetch_aside(tensors, nbytes_each: int):
-    """Start pulling the first ``nbytes_each`` bytes of every tensor into L2 on the side stream (forked from the current stream at
-    this point, NOT joined here: nothing depends on a prefetch — :func:`join_aside` ties the side stream back once per forward so
-    a graph capture ends with all its branches joined).  The main stream's kernel chain keeps its programmatic (PDL) edges."""
-    cur = torch.cuda.current_stream()
-    dev = cur.device.index
-    side = _side_streams.get(dev)
-    if side is None:
-        side = _side_streams[dev] = torch.cuda.Stream(device=cur.device)
-    fork = torch.cuda.Event()
-    fork.record(cur)
-    side.wait_event(fork)
-    with torch.cuda.stream(side):
-        for t in tensors:
-            C().l2_prefetch(t, 0, min(int(nbytes_each), t.numel() * t.element_size()) // 16 * 16)
-        done = torch.cuda.Event()
-        done.record(side)
-    _aside_last[dev] = done
-
-
-def join_aside():
-    """Join the side stream's outstanding prefetches into the current stream (end of a forward pass)."""
-    cur = torch.cuda.current_stream()
-    ev = _aside_last.pop(cur.device.index, None)
-    if ev is not None:
-        cur.wait_event(ev)
-        C().pdl_skip_next()
-
-
-def l2_prefetch_bytes() -> int:
-    """Bytes of the next MoE block's gate / up banks (each) to prefetch into L2 during a decode layer's attention chain
-    (``MLXB200_L2_PREFETCH_MB``, total across both banks; 0 = off)."""
-    try:
-        return int(float(os.environ.get("MLXB200_L2_PREFETCH_MB", "0")) * (1 << 20)) // 2
-    except ValueError:
-        return 0
-
-
 def moe_experts(x, idx, w, Wg: LinearWeight, Wu: LinearWeight, Wd: LinearWeight, act: str = "silu",
                 extra: Optional[torch.Tensor] = None, residual: Optional[torch.Tensor] = None,
                 out: Optional[torch.Tensor] = None, signal: Optional[Tuple[int, int]] = None, join: Optional[_Join] = None):
@@ -279,7 +243,9 @@ def moe_experts(x, idx, w, Wg: LinearWeight, Wu: LinearWeight, Wd: LinearWeight,
     weighted combine (+ residual [+ P2P store & flag])."""
     c = C()
     T, k = idx.shape
-    if fp8_experts_enabled(Wg) and x.shape[1] % 128 == 0:
+    fp8 = fp8_experts_enabled(Wg) and x.shape[1] % 128 == 0
+    qg, qu, qd = (None, None, None) if fp8 else (_qpack(Wg), _qpack(Wu), _qpack(Wd))
+    if fp8:
         (gq, gs), (uq, us), (dq, ds) = _fp8pack(Wg), _fp8pack(Wu), _fp8pack(Wd)
         E = gq.shape[0]
         offs, pair_row, xp = c.moe_permute(idx, x, E)
@@ -287,14 +253,7 @@ def moe_experts(x, idx, w, Wg: LinearWeight, Wu: LinearWeight, Wd: LinearWeight,
         h = c.linear_fp8(xq, xsf, gq, gs, uq, us, offs, T, None, ACT_IDS[act], False, 0, 0)
         hq, hsf = c.quant_mxfp8(h)
         y = c.linear_fp8(hq, hsf, dq, ds, None, None, offs, T, None, 0, True, 0, 0)
-        if extra is not None:
-            residual = extra if residual is None else residual + extra
-        flag, val = signal if signal is not None else (0, 0)
-        if join is not None:
-            join.wait()
-        return c.moe_combine(y, pair_row, w, residual, out, int(k), int(flag), int(val))
-    qg, qu, qd = _qpack(Wg), _qpack(Wu), _qpack(Wd)
-    if qg is not None and qu is not None and qd is not None:
+    elif qg is not None and qu is not None and qd is not None:
         E = Wg.wq.shape[0]
         offs, pair_row, xp = c.moe_permute(idx, x, E)
         h = c.grouped_linear_q(xp, qg[0], qg[1], qg[2], qu[0], qu[1], qu[2], Wg.bits, Wg.group_size, E, Wg.out_features,
@@ -361,23 +320,22 @@ def moe_block(x, gate_w, route_kw: dict, Wg: LinearWeight, Wu: LinearWeight, Wd:
     the scatter path the router kernel normalises the row in shared memory (no norm kernel).  ``next_norm = (weight, eps)``: the
     block also returns ``rmsnorm(result) * weight`` (the next layer's input norm), fused into the combine kernel on the scatter
     path; the return value is then ``(result, normed)``.
-  Decode-sized batches with bf16 banks take the *scatter*
-    path: the router kernel claims a slot per (token, expert) pair in the expert's fixed-stride segment and copies the token row
-    there itself, the grouped GEMMs read per-expert row counts — route / counting sort / gather are ONE launch, the block is
-    router -> grouped gate-up -> grouped down -> combine.  Larger batches (prefill) keep the compact counting-sort permutation."""
+
+    Decode-sized batches (``T <= SCATTER_MAX_TOKENS``) with bf16 or FP8 banks take the *scatter* path: the router kernel claims a
+    slot per (token, expert) pair in the expert's fixed-stride segment and copies the token row there itself, the grouped GEMMs
+    read per-expert row counts — route / counting sort / gather are ONE launch, the block is router -> grouped gate-up -> grouped
+    down -> combine.  Larger batches (prefill) and packed-integer banks keep the compact counting-sort permutation, with the
+    norms as separate kernels."""
     c = C()
     T = x.shape[0]
     fp8 = fp8_experts_enabled(Wg) and x.shape[1] % 128 == 0
     quant = (Wg.is_quantized or Wu.is_quantized or Wd.is_quantized) and not fp8
-    if quant or T > SCATTER_MAX_TOKENS or os.environ.get("MLXB200_MOE_SCATTER", "1") == "0":
+    if quant or T > SCATTER_MAX_TOKENS:
         if pre_norm is not None:
             x = rmsnorm(x, pre_norm[0], pre_norm[1])
         idx, wts = moe_route(x, gate_w, extra=extra, **route_kw)
         res = moe_experts(x, idx, wts, Wg, Wu, Wd, act, residual=residual, out=out, signal=signal)
         return res if next_norm is None else (res, rmsnorm(res, next_norm[0], next_norm[1]))
-    fuse_norms = os.environ.get("MLXB200_FUSE_NORMS", "1") != "0"
-    if pre_norm is not None and not fuse_norms:
-        x, pre_norm = rmsnorm(x, pre_norm[0], pre_norm[1]), None
     if fp8:
         (gq, gs), (uq, us), (dq, ds) = _fp8pack(Wg), _fp8pack(Wu), _fp8pack(Wd)
         E, H = gq.shape[0], x.shape[1]
@@ -392,12 +350,10 @@ def moe_block(x, gate_w, route_kw: dict, Wg: LinearWeight, Wu: LinearWeight, Wd:
         bufs = _scatter_bufs[key] = (torch.zeros(E, dtype=torch.int32, device=x.device),
                                      torch.empty(E * stride, H, dtype=torch.bfloat16, device=x.device))
     counts, xs = bufs
-    rk = dict(route_kw)
-    method = rk.pop("method", "greedy")
-    if method != "group_limited_greedy":
-        rk["n_group"], rk["topk_group"] = 1, 1
+    rk = route_kw
+    n_group, topk_group = route_groups(rk.get("method", "greedy"), rk.get("n_group", 1), rk.get("topk_group", 1))
     nw, ne = (_bf16(pre_norm[0]), float(pre_norm[1])) if pre_norm is not None else (None, 1e-6)
-    idx, wts, pair_row = c.moe_route(x, _bf16(gate_w), int(rk["top_k"]), int(rk["n_group"]), int(rk["topk_group"]), float(rk["scaling"]),
+    idx, wts, pair_row = c.moe_route(x, _bf16(gate_w), int(rk["top_k"]), n_group, topk_group, float(rk["scaling"]),
                                      bool(rk["norm_topk"]), int(extra), counts, stride, xs, nw, ne)
     k = idx.shape[1]
     if fp8:
@@ -411,7 +367,7 @@ def moe_block(x, gate_w, route_kw: dict, Wg: LinearWeight, Wu: LinearWeight, Wd:
         h = c.grouped_linear(xs, wg, wu, counts, stride, ACT_IDS[act], False, None, None, None, T * k, stride)
         y = c.grouped_linear(h, wd, None, counts, stride, 0, True, None, None, None, T * k, stride)
     flag, val = signal if signal is not None else (0, 0)
-    if next_norm is not None and signal is None and fuse_norms and H <= 8192:
+    if next_norm is not None and signal is None and H <= 8192:   # (the fused combine-norm kernel holds a row of up to 8192)
         normed = torch.empty(T, H, dtype=torch.bfloat16, device=x.device)
         res = c.moe_combine(y, pair_row, wts, residual, out, int(k), 0, 0, counts, _bf16(next_norm[0]), float(next_norm[1]), normed)
         return res, normed

@@ -291,12 +291,6 @@ void rope_(Tensor x, const Tensor& positions, const Tensor& inv_freq, int64_t ro
                             (int)rot_off, (int)rot_dim, interleaved, (float)mscale, (int)x.size(0), cur_stream()));
 }
 
-void l2_prefetch(const Tensor& t, int64_t offset_bytes, int64_t nbytes) {
-  TORCH_CHECK(t.is_cuda() && t.is_contiguous() && offset_bytes >= 0 && nbytes >= 0 && offset_bytes + nbytes <= (int64_t)t.nbytes(), "bad prefetch range");
-  const c10::cuda::CUDAGuard guard(t.device());
-  LAUNCH_OK(b200::l2_prefetch_launch(static_cast<const char*>(t.data_ptr()) + offset_bytes, (unsigned long long)nbytes, cur_stream()));
-}
-
 Tensor embed(const Tensor& ids, const Tensor& table, const c10::optional<Tensor>& scales, const c10::optional<Tensor>& biases,
              int64_t bits, int64_t group, double scale) {
   TORCH_CHECK(ids.is_cuda() && ids.scalar_type() == torch::kInt64 && ids.is_contiguous(), "ids must be contiguous int64 CUDA");
@@ -682,21 +676,6 @@ std::vector<unsigned long long> to_u64(const std::vector<int64_t>& v) {
   for (size_t i = 0; i < v.size(); ++i) o[i] = (unsigned long long)v[i];
   return o;
 }
-void ep_dispatch(const Tensor& x, const Tensor& idx, int64_t experts_per_rank, int64_t my_rank, int64_t cap,
-                 std::vector<int64_t> recv_x, std::vector<int64_t> recv_meta, std::vector<int64_t> recv_words, Tensor send_seq,
-                 Tensor send_counts, Tensor done_counter, const c10::optional<Tensor>& ret_expected) {
-  check_bf16(x, "x"); check_rows(x, "x");
-  TORCH_CHECK(idx.scalar_type() == torch::kInt32 && idx.is_contiguous() && idx.dim() == 2);
-  const c10::cuda::CUDAGuard guard(x.device());
-  const int world = (int)recv_x.size();
-  auto a = to_u64(recv_x), b = to_u64(recv_meta), c = to_u64(recv_words);
-  LAUNCH_OK(b200::ep_dispatch_launch(x.data_ptr(), x.stride(0), idx.data_ptr<int>(), (int)idx.numel(), (int)idx.size(1), (int)x.size(1),
-                                     (int)experts_per_rank, world, (int)my_rank, (int)cap, a.data(), b.data(), c.data(),
-                                     reinterpret_cast<uint32_t*>(send_seq.data_ptr<int>()), send_counts.data_ptr<int>(),
-                                     reinterpret_cast<unsigned int*>(done_counter.data_ptr<int>()),
-                                     ret_expected.has_value() ? reinterpret_cast<uint32_t*>(ret_expected->data_ptr<int>()) : nullptr,
-                                     cur_stream()));
-}
 void ep_dispatch_scatter(const Tensor& x, const Tensor& idx, int64_t experts_per_rank, int64_t my_rank, int64_t cap_e,
                          std::vector<int64_t> recv_x, std::vector<int64_t> recv_dst, std::vector<int64_t> recv_cnt,
                          std::vector<int64_t> recv_seq, std::vector<int64_t> my_ret, Tensor send_seq, Tensor done_counter,
@@ -714,7 +693,7 @@ void ep_dispatch_scatter(const Tensor& x, const Tensor& idx, int64_t experts_per
                                              cur_stream()));
 }
 
-// Router + expert-parallel dispatch in one kernel (v2 exchange): returns {idx, wts}; optionally normalises `x` first (norm_w) and
+// Router + expert-parallel dispatch in one kernel: returns {idx, wts}; optionally normalises `x` first (norm_w) and
 // stores the normalised rows (normed_out) for the shared-expert branch.
 std::vector<Tensor> ep_route_dispatch(const Tensor& x, const Tensor& gate_w, int64_t top_k, int64_t n_group, int64_t topk_group, double scaling,
                                       bool norm_topk, int64_t experts_per_rank, int64_t my_rank, int64_t cap_e, std::vector<int64_t> recv_x,
@@ -748,30 +727,6 @@ std::vector<Tensor> ep_route_dispatch(const Tensor& x, const Tensor& gate_w, int
   return {idx, w};
 }
 
-std::vector<Tensor> ep_regroup(int64_t recv_words_ptr, int64_t counter_ptr, int64_t error_ptr, int64_t recv_meta_ptr,
-                               int64_t recv_x_ptr, int64_t world, int64_t cap, int64_t E_local, int64_t H, int64_t device,
-                               int64_t rows_bound, std::vector<int64_t> ret_y) {
-  auto dev = torch::Device(torch::kCUDA, (int)device);
-  const c10::cuda::CUDAGuard guard(dev);
-  auto io = torch::dtype(torch::kInt32).device(dev);
-  // rows_bound (>0): the caller's bound on the rows all sources can send this step; sizes the expert-ordered temporaries
-  const int64_t R = rows_bound > 0 ? std::min<int64_t>(world * cap, rows_bound) : world * cap;
-  Tensor offs = torch::empty({E_local + 1}, io), row_perm = torch::empty({world * cap}, io), total = torch::empty({1}, io);
-  Tensor counts = torch::empty({world}, io);
-  Tensor x_perm = torch::empty({R, H}, torch::dtype(torch::kBFloat16).device(dev));
-  // destination address of every expert-ordered row for the fused return (down-projection epilogue -> source's return buffer)
-  Tensor row_dst = torch::empty({ret_y.empty() ? 0 : R}, torch::dtype(torch::kInt64).device(dev));
-  auto ry = to_u64(ret_y);
-  LAUNCH_OK(b200::ep_regroup_launch(reinterpret_cast<const unsigned long long*>(recv_words_ptr), reinterpret_cast<uint32_t*>(counter_ptr),
-                                    reinterpret_cast<uint32_t*>(error_ptr), counts.data_ptr<int>(),
-                                    reinterpret_cast<const void*>(recv_meta_ptr), reinterpret_cast<const void*>(recv_x_ptr), (int)world,
-                                    (int)cap, (int)E_local, (int)H, offs.data_ptr<int>(), row_perm.data_ptr<int>(), total.data_ptr<int>(),
-                                    x_perm.data_ptr(), ret_y.empty() ? nullptr : ry.data(),
-                                    ret_y.empty() ? nullptr : reinterpret_cast<unsigned long long*>(row_dst.data_ptr<int64_t>()),
-                                    cur_stream()));
-  ++g_launches;
-  return {offs, total, x_perm, row_dst};
-}
 Tensor ep_combine(int64_t flag_ptr, const Tensor& expected, int64_t error_ptr, const Tensor& ret_y, const Tensor& wts,
                   const c10::optional<Tensor>& residual, const c10::optional<Tensor>& out_, const c10::optional<Tensor>& norm_w,
                   double norm_eps, const c10::optional<Tensor>& normed) {
@@ -812,7 +767,6 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("rmsnorm", &rmsnorm, py::arg("x"), py::arg("w"), py::arg("eps"), py::arg("gemma") = false, py::arg("residual") = py::none(),
         py::arg("out") = py::none(), py::arg("signal_flag_ptr") = 0, py::arg("signal_value") = 0);
   m.def("rope_", &rope_);
-  m.def("l2_prefetch", &l2_prefetch, py::arg("t"), py::arg("offset_bytes"), py::arg("nbytes"));
   m.def("embed", &embed, py::arg("ids"), py::arg("table"), py::arg("scales") = py::none(), py::arg("biases") = py::none(),
         py::arg("bits") = 0, py::arg("group") = 64, py::arg("scale") = 1.0);
   m.def("kv_write", &kv_write);
@@ -850,15 +804,9 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("set_flag", &set_flag);
   m.def("copy_signal", &copy_signal);
   m.def("advance_meta", &advance_meta);
-  m.def("ep_dispatch", &ep_dispatch, py::arg("x"), py::arg("idx"), py::arg("experts_per_rank"), py::arg("my_rank"), py::arg("cap"),
-        py::arg("recv_x"), py::arg("recv_meta"), py::arg("recv_words"), py::arg("send_seq"), py::arg("send_counts"),
-        py::arg("done_counter"), py::arg("ret_expected") = py::none());
   m.def("ep_dispatch_scatter", &ep_dispatch_scatter, py::arg("x"), py::arg("idx"), py::arg("experts_per_rank"), py::arg("my_rank"),
         py::arg("cap_e"), py::arg("recv_x"), py::arg("recv_dst"), py::arg("recv_cnt"), py::arg("recv_seq"), py::arg("my_ret"),
         py::arg("send_seq"), py::arg("done_counter"), py::arg("ret_expected") = py::none());
-  m.def("ep_regroup", &ep_regroup, py::arg("recv_words_ptr"), py::arg("counter_ptr"), py::arg("error_ptr"),
-        py::arg("recv_meta_ptr"), py::arg("recv_x_ptr"), py::arg("world"), py::arg("cap"), py::arg("E_local"), py::arg("H"),
-        py::arg("device"), py::arg("rows_bound") = 0, py::arg("ret_y") = std::vector<int64_t>());
   m.def("ep_combine", &ep_combine, py::arg("flag_ptr"), py::arg("expected"), py::arg("error_ptr"), py::arg("ret_y"), py::arg("wts"),
         py::arg("residual") = py::none(), py::arg("out") = py::none(), py::arg("norm_w") = py::none(), py::arg("norm_eps") = 1e-6,
         py::arg("normed") = py::none());

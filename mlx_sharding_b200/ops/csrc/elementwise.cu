@@ -251,27 +251,6 @@ __global__ void embed_quant_kernel(const long long* __restrict__ ids, const uint
   }
 }
 
-// ------------------------------------------------------------------------------------------------ L2 prefetch
-// Pulls a weight range into the 126 MB L2 with bulk prefetches (no SM registers / shared memory involved, a handful of threads).
-// Launched on a side stream while the latency-bound attention chain of a decode layer leaves HBM idle, for the first experts of the
-// MoE bank the following grouped GEMM streams: that GEMM is HBM-bound, so every byte already in L2 comes off its critical path.
-__global__ void l2_prefetch_kernel(const char* __restrict__ p, unsigned long long bytes) {
-  constexpr unsigned long long kChunk = 8192;
-  const unsigned long long step = (unsigned long long)gridDim.x * blockDim.x * kChunk;
-  for (unsigned long long i = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) * kChunk; i < bytes; i += step) {
-    const unsigned long long left = bytes - i;
-    const unsigned int n = (unsigned int)(left < kChunk ? (left & ~15ull) : kChunk);
-    if (n) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p + i), "r"(n) : "memory");
-  }
-}
-
-cudaError_t l2_prefetch_launch(const void* p, unsigned long long bytes, cudaStream_t s) {
-  if (bytes == 0) return cudaSuccess;
-  if (reinterpret_cast<uintptr_t>(p) & 15) return cudaErrorInvalidValue;
-  l2_prefetch_kernel<<<8, 128, 0, s>>>(static_cast<const char*>(p), bytes);
-  return cudaGetLastError();
-}
-
 cudaError_t embed_launch(const long long* ids, const void* table, const void* scales, const void* biases, int bits, int group,
                          void* out, int H, float scale, int T, cudaStream_t s) {
   if (T == 0) return cudaSuccess;

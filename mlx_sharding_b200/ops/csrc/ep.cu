@@ -2,23 +2,24 @@
 //
 // The reference keeps all 64 routed experts of a layer on one stage (`mx.gather_qmm`); there is no
 // collective anywhere in it.  Here the experts of every MoE layer can be sharded across the ranks of one
-// NVSwitch domain and the token exchange is done by our own kernels — no NCCL call, no host hop:
+// NVSwitch domain and the token exchange is done by our own kernels in four launches — no NCCL call, no host hop:
 //
-//   dispatch  : every (token, k) pair whose expert lives on rank r is written *directly* into r's receive
-//               region for this source (peer-mapped memory, 16 B stores), together with a (local expert,
-//               source pair) record; the last CTA publishes (row count << 32 | step sequence) to each destination
-//               as one 64-bit st.release.sys.
-//   regroup   : the destination polls the W words (ld.acquire.sys), buckets what it received by local expert
-//               (offsets + gather) so the swap-AB grouped tcgen05 GEMMs run on contiguous rows, and records for
-//               every row the address of its slot in the source rank's return buffer.
-//   return    : there is no return kernel — the grouped down-projection's epilogue (gemm_persistent.cu, GemmParams::
-//               row_dst / signal_peers) stores each fp32 output row straight to that address and the CTA completing the
-//               grid bumps every source's flag.
-//   combine   : the source waits (in-kernel) for all W arrivals, then does the weighted combine (+ residual).
+//   dispatch  : slot reservation at the sender.  Every (token, k) pair claims a row in its owner's expert-major receive
+//               buffer with one system-scope atomic on the owner's per-expert row counter, stores the token row there
+//               (peer-mapped memory, 16 B stores) together with the address of the pair's slot in the sender's return
+//               buffer; the last CTA publishes the step's sequence number to every destination (st.release.sys).
+//               ep_dispatch_scatter_kernel below, or the router with the dispatch folded in (moe.cu, RouteEP).
+//   gate/up   : the grouped swap-AB tcgen05 GEMM on the receive buffer; its CTAs first acquire every source's sequence
+//               word (gemm_persistent.cu, GemmParams::ep_arrive), so the arrival wait needs no kernel of its own.
+//   down      : the grouped down-projection's epilogue (GemmParams::row_dst / signal_peers) stores each fp32 output row
+//               straight to its return address and the CTA completing the grid bumps every source's flag.
+//   combine   : the source waits (in-kernel) for all W arrivals, then does the weighted combine (+ residual, optionally
+//               + the next layer's input RMSNorm).
 //
-// Sequence numbers / counting flags + device-resident expectations make every step CUDA-graph replay safe.  Buffer
-// reuse is race-free by construction: a source only dispatches layer l+1 after it has combined layer l, which
-// requires every destination to have regrouped (consumed) layer l and returned its rows.
+// Sequence numbers / counting flags + device-resident expectations make every step CUDA-graph replay safe; the per-expert
+// row counters are double-buffered by step parity and the gate/up GEMM clears the other parity's.  Buffer reuse is race-free
+// by construction: a source only dispatches layer l+1 after it has combined layer l, which requires every destination to have
+// run its down-projection (consumed its receive buffer) for layer l and returned its rows.
 #include "kernels.h"
 #include "launch.h"
 #include "ptx.cuh"
@@ -31,66 +32,9 @@ constexpr int kMaxWorld = kEpMaxWorld;
 using PeerTable = EpPeerTable;
 
 // ---------------------------------------------------------------------------------------------- dispatch
-// one warp per (token, k) pair
-__global__ void ep_dispatch_kernel(const __nv_bfloat16* __restrict__ x, long long ld_x, const int* __restrict__ idx, int npairs,
-                                   int top_k, int H, int experts_per_rank, int world, int my_rank, int cap,
-                                   PeerTable recv_x,      // per dst: base of [world][cap][H] bf16 (its receive regions)
-                                   PeerTable recv_meta,   // per dst: base of [world][cap] int2
-                                   PeerTable recv_count,  // per dst: base of [world] u64 words (count << 32 | step sequence)
-                                   uint32_t* __restrict__ send_seq,  // my step sequence number (device resident)
-                                   int* __restrict__ send_counts, unsigned int* __restrict__ done_counter,
-                                   uint32_t* __restrict__ ret_expected /* += world: arrivals the combine of this step waits for */) {
-  pdl_sync();  // PDL: predecessor's writes visible; let the successor start its prologue
-  const int warps_per_cta = blockDim.x >> 5;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int nvec = H / 8;
-  for (int p = blockIdx.x * warps_per_cta + warp; p < npairs; p += gridDim.x * warps_per_cta) {
-    const int e = idx[p];
-    const int dst = e / experts_per_rank;
-    int slot = 0;
-    if (lane == 0) slot = atomicAdd(&send_counts[dst], 1);
-    slot = __shfl_sync(0xffffffffu, slot, 0);
-    if (slot < cap) {
-      const uint4* src = reinterpret_cast<const uint4*>(x + (size_t)(p / top_k) * ld_x);
-      uint4* drow = reinterpret_cast<uint4*>(recv_x.p[dst]) + ((size_t)my_rank * cap + slot) * nvec;
-      for (int v = lane; v < nvec; v += 32) drow[v] = src[v];
-      if (lane == 0) {
-        int2* m = reinterpret_cast<int2*>(recv_meta.p[dst]) + (size_t)my_rank * cap + slot;
-        *m = make_int2(e - dst * experts_per_rank, p);
-      }
-    }
-  }
-  // publish: the last CTA tells every destination how many rows it got from me.  Count and step sequence number travel in ONE
-  // 64-bit word written with st.release.sys (every CTA fenced its row stores before arriving on done_counter), so the
-  // receiver needs no separate flag and the sender no second fence / atomic round trip.
-  __threadfence_system();
-  __syncthreads();
-  __shared__ bool last;
-  if (threadIdx.x == 0) last = (atomicAdd(done_counter, 1u) + 1u == gridDim.x);
-  __syncthreads();
-  if (last) {
-    __threadfence_system();
-    const uint32_t seq = *send_seq + 1u;
-    for (int r = threadIdx.x; r < world; r += blockDim.x) {
-      int c = __ldcg(&send_counts[r]);
-      if (c > cap) c = cap;
-      send_counts[r] = 0;
-      st_release_sys_u64(reinterpret_cast<unsigned long long*>(recv_count.p[r]) + my_rank,
-                         (static_cast<unsigned long long>(static_cast<uint32_t>(c)) << 32) | seq);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      *send_seq = seq;
-      *done_counter = 0u;
-      if (ret_expected != nullptr) *ret_expected += (uint32_t)world;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------- dispatch, v2 (scatter)
 // Sender-side slot reservation: each (token, k) pair claims a slot in the *destination's* expert-major receive buffer with one
 // system-scope atomic on the destination's per-expert row counter (counters double-buffered by step parity), so rows land
-// expert-contiguous where the grouped GEMM's TMA reads them — the receiver needs no regroup (counting sort + gather) kernels.
+// expert-contiguous where the grouped GEMM's TMA reads them and the receiver needs no counting sort or gather of its own.
 // Next to the row the sender stores the address of the pair's slot in ITS return buffer *as mapped by the destination* (table
 // exchanged at set-up), which is what the down-projection epilogue stores to.  Publication: the last CTA writes the step's sequence
 // number to every destination (release.sys, after every CTA fenced its rows); the destination's grouped GEMM acquires all of them
@@ -139,77 +83,6 @@ __global__ void ep_dispatch_scatter_kernel(const __nv_bfloat16* __restrict__ x, 
       *send_seq = seq;
       *done_counter = 0u;
       if (ret_expected != nullptr) *ret_expected += (uint32_t)world;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------- regroup
-// single CTA: wait for all sources, bucket received rows by local expert
-__global__ void __launch_bounds__(1024)
-ep_regroup_offsets_kernel(const unsigned long long* recv_words, uint32_t* local_counter, uint32_t* error_flag, unsigned long long timeout_ns,
-                          int* __restrict__ recv_count_out, const int2* __restrict__ recv_meta, int world, int cap,
-                          int E_local, int* __restrict__ expert_offsets, int* __restrict__ row_perm /*[world*cap]*/,
-                          int* __restrict__ total_rows) {
-  pdl_sync();  // PDL: predecessor's writes visible; let the successor start its prologue
-  __shared__ int cnt[256], cur[256];
-  __shared__ int counts[kMaxWorld];
-  __shared__ uint32_t expected_s;
-  if (threadIdx.x == 0) expected_s = *local_counter + 1u;   // my own step sequence number
-  __syncthreads();
-  if (threadIdx.x < world) {
-    // source `threadIdx.x` publishes (count << 32 | seq) once its rows are visible: poll until it carries this step's seq
-    const uint32_t expected = expected_s;
-    const unsigned long long* word = recv_words + threadIdx.x;
-    unsigned long long t0, v;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0));
-    while (true) {
-      v = ld_acquire_sys_u64(word);
-      if (static_cast<uint32_t>(v) == expected) break;
-      unsigned long long t1;
-      asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t1));
-      if (t1 - t0 > timeout_ns) { if (error_flag) atomicExch(error_flag, 1u); v = 0; break; }
-      __nanosleep(32);
-    }
-    counts[threadIdx.x] = static_cast<int>(v >> 32);
-    recv_count_out[threadIdx.x] = counts[threadIdx.x];   // plain copy for the gather kernel
-    __threadfence_system();
-  }
-  if (threadIdx.x == 0) *local_counter = expected_s;
-  for (int e = threadIdx.x; e < E_local; e += blockDim.x) cnt[e] = 0;
-  __syncthreads();
-  for (int s = 0; s < world; ++s)
-    for (int j = threadIdx.x; j < counts[s]; j += blockDim.x) atomicAdd(&cnt[__ldcv(&recv_meta[(size_t)s * cap + j].x)], 1);
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int acc = 0;
-    for (int e = 0; e < E_local; ++e) { cur[e] = acc; expert_offsets[e] = acc; acc += cnt[e]; }
-    expert_offsets[E_local] = acc;
-    *total_rows = acc;
-  }
-  __syncthreads();
-  for (int s = 0; s < world; ++s)
-    for (int j = threadIdx.x; j < counts[s]; j += blockDim.x)
-      row_perm[(size_t)s * cap + j] = atomicAdd(&cur[__ldcv(&recv_meta[(size_t)s * cap + j].x)], 1);
-}
-
-// gather received rows into expert-contiguous order; remember where each permuted row came from
-__global__ void ep_regroup_gather_kernel(const __nv_bfloat16* __restrict__ recv_x, const int2* __restrict__ recv_meta,
-                                         const int* __restrict__ recv_count, const int* __restrict__ row_perm, int world, int cap,
-                                         int H, __nv_bfloat16* __restrict__ x_perm, PeerTable ret_y,
-                                         unsigned long long* __restrict__ row_dst /*fp32 return row of each permuted row*/) {
-  pdl_sync();  // PDL: predecessor's writes visible; let the successor start its prologue
-  const int nvec = H / 8;
-  const int s = blockIdx.y;
-  const int n = recv_count[s];
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < (long long)n * nvec; i += (long long)gridDim.x * blockDim.x) {
-    const int j = i / nvec, v = i % nvec;
-    const int row = row_perm[(size_t)s * cap + j];
-    reinterpret_cast<uint4*>(x_perm + (size_t)row * H)[v] =
-        __ldcv(reinterpret_cast<const uint4*>(recv_x + ((size_t)s * cap + j) * H) + v);
-    if (v == 0) {
-      const int pair = recv_meta[(size_t)s * cap + j].y;
-      // where the down-projection epilogue stores this row: the source rank's return buffer, at the pair's index
-      if (row_dst != nullptr) row_dst[row] = ret_y.p[s] + (unsigned long long)pair * (unsigned long long)H * sizeof(float);
     }
   }
 }
@@ -386,20 +259,6 @@ PeerTable make_table(const unsigned long long* v, int world) {
 
 }  // namespace
 
-cudaError_t ep_dispatch_launch(const void* x, long long ld_x, const int* idx, int npairs, int top_k, int H, int experts_per_rank,
-                               int world, int my_rank, int cap, const unsigned long long* recv_x, const unsigned long long* recv_meta,
-                               const unsigned long long* recv_count, uint32_t* send_seq, int* send_counts,
-                               unsigned int* done_counter, uint32_t* ret_expected, cudaStream_t s) {
-  if (world > kMaxWorld || (H % 8)) return cudaErrorInvalidValue;
-  int grid = (npairs + 7) / 8;
-  if (grid < 1) grid = 1;
-  if (grid > 592) grid = 592;
-  (void)launch_pdl(ep_dispatch_kernel, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(x), ld_x, idx, npairs, top_k, H, experts_per_rank, world,
-                                          my_rank, cap, make_table(recv_x, world), make_table(recv_meta, world),
-                                          make_table(recv_count, world), send_seq, send_counts, done_counter, ret_expected);
-  return cudaGetLastError();
-}
-
 cudaError_t ep_dispatch_scatter_launch(const void* x, long long ld_x, const int* idx, int npairs, int top_k, int H, int experts_per_rank,
                                        int world, int my_rank, int cap_e, const unsigned long long* recv_x,
                                        const unsigned long long* recv_dst, const unsigned long long* recv_cnt,
@@ -413,23 +272,6 @@ cudaError_t ep_dispatch_scatter_launch(const void* x, long long ld_x, const int*
                    experts_per_rank, world, my_rank, cap_e, make_table(recv_x, world), make_table(recv_dst, world),
                    make_table(recv_cnt, world), make_table(recv_seq, world), make_table(my_ret, world), send_seq, done_counter,
                    ret_expected);
-  return cudaGetLastError();
-}
-
-cudaError_t ep_regroup_launch(const unsigned long long* recv_words, uint32_t* local_counter, uint32_t* error_flag, int* recv_count,
-                              const void* recv_meta, const void* recv_x, int world, int cap, int E_local, int H, int* expert_offsets,
-                              int* row_perm, int* total_rows, void* x_perm, const unsigned long long* ret_y,
-                              unsigned long long* row_dst, cudaStream_t s) {
-  if (E_local > 256 || world > kMaxWorld) return cudaErrorInvalidValue;
-  (void)launch_pdl(ep_regroup_offsets_kernel, dim3(1), dim3(1024), 0, s, recv_words, local_counter, error_flag, kTimeoutNs, recv_count,
-                                               static_cast<const int2*>(recv_meta), world, cap, E_local, expert_offsets, row_perm,
-                                               total_rows);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return e;
-  dim3 grid(64, world);
-  (void)launch_pdl(ep_regroup_gather_kernel, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(recv_x), static_cast<const int2*>(recv_meta), static_cast<const int*>(recv_count),
-                                                row_perm, world, cap, H, static_cast<__nv_bfloat16*>(x_perm),
-                                                ret_y != nullptr ? make_table(ret_y, world) : PeerTable{}, row_dst);
   return cudaGetLastError();
 }
 

@@ -12,8 +12,6 @@ cudaError_t rmsnorm_launch(const void* x, long long ld_x, const void* w, const v
                            uint32_t signal_value = 0, unsigned int* done_counter = nullptr);
 cudaError_t rope_launch(void* x, long long ld_t, long long ld_h, int heads, const int* positions, const float* inv_freq,
                         int rot_off, int rot_dim, bool interleaved, float mscale, int T, cudaStream_t s);
-// bulk L2 prefetch of [p, p + bytes) (16 B aligned), a few threads, no PDL: meant for a side stream
-cudaError_t l2_prefetch_launch(const void* p, unsigned long long bytes, cudaStream_t s);
 cudaError_t embed_launch(const long long* ids, const void* table, const void* scales, const void* biases, int bits, int group,
                          void* out, int H, float scale, int T, cudaStream_t s);
 cudaError_t kv_write_launch(const void* k, long long k_ld_t, long long k_ld_h, const void* v, long long v_ld_t,
@@ -73,7 +71,7 @@ constexpr int kEpMaxWorld = 16;
 struct EpPeerTable {
   unsigned long long p[kEpMaxWorld];
 };
-// Fused router + expert-parallel dispatch (v2 exchange, see ep.cu): the router CTA of a token reserves the slots of its top-k pairs
+// Fused router + expert-parallel dispatch (see ep.cu): the router CTA of a token reserves the slots of its top-k pairs
 // in the owners' expert-major receive buffers (remote atomics), stores the (normalised) row there and takes part in the
 // publication protocol of ep_dispatch_scatter_kernel — one kernel instead of norm + route + dispatch.
 struct RouteEP {
@@ -133,20 +131,12 @@ cudaError_t advance_meta_launch(int* positions, int* context_lens, int* slots, c
 void pdl_skip_next();
 
 // ---- ep.cu (expert-parallel all-to-all over peer memory)
-cudaError_t ep_dispatch_launch(const void* x, long long ld_x, const int* idx, int npairs, int top_k, int H, int experts_per_rank,
-                               int world, int my_rank, int cap, const unsigned long long* recv_x, const unsigned long long* recv_meta,
-                               const unsigned long long* recv_count, uint32_t* send_seq, int* send_counts,
-                               unsigned int* done_counter, uint32_t* ret_expected, cudaStream_t s);
-// v2: sender-side slot reservation into the destination's expert-major buffer (no regroup kernels on the receive side)
+// dispatch: sender-side slot reservation into each destination's expert-major receive buffer
 cudaError_t ep_dispatch_scatter_launch(const void* x, long long ld_x, const int* idx, int npairs, int top_k, int H, int experts_per_rank,
                                        int world, int my_rank, int cap_e, const unsigned long long* recv_x,
                                        const unsigned long long* recv_dst, const unsigned long long* recv_cnt,
                                        const unsigned long long* recv_seq, const unsigned long long* my_ret, uint32_t* send_seq,
                                        unsigned int* done_counter, uint32_t* ret_expected, cudaStream_t s);
-cudaError_t ep_regroup_launch(const unsigned long long* recv_words, uint32_t* local_counter, uint32_t* error_flag, int* recv_count,
-                              const void* recv_meta, const void* recv_x, int world, int cap, int E_local, int H, int* expert_offsets,
-                              int* row_perm, int* total_rows, void* x_perm, const unsigned long long* ret_y,
-                              unsigned long long* row_dst, cudaStream_t s);
 cudaError_t ep_combine_launch(const uint32_t* flag, const uint32_t* expected_ptr, uint32_t* error_flag, const float* ret_y,
                               const float* wts, const void* residual, long long ld_res, void* out, long long ld_out, int T, int top_k,
                               int H, cudaStream_t s, const void* norm_w = nullptr, float norm_eps = 0.f,

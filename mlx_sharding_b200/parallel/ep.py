@@ -23,11 +23,13 @@ from ..ops.weights import LinearWeight
 
 
 class EPBuffers:
-    """IPC-mapped receive / return buffers of one rank (shared by all MoE layers of that rank)."""
+    """IPC-mapped receive / return buffers of one rank (shared by all MoE layers of that rank).
 
-    def __init__(self, hidden: int, max_tokens: int, top_k: int, group=None, experts_per_rank: int = 0):
-        import os
+    Receive side: an expert-major buffer of ``[experts_per_rank][world * max_tokens][H]`` bf16 rows, the return address of every
+    row (u64), two parity-buffered sets of per-expert row counters and one arrival word per source.  Return side: ``[max_tokens *
+    top_k][H]`` fp32 rows (one per routed pair of this rank) and the return flag."""
 
+    def __init__(self, hidden: int, max_tokens: int, top_k: int, experts_per_rank: int, group=None):
         from ..ops import b200
 
         self.C = b200.load_extension()
@@ -35,23 +37,15 @@ class EPBuffers:
         self.dev = torch.cuda.current_device()
         self.H, self.top_k = hidden, top_k
         self.max_tokens = max_tokens
-        # v2 (default): sender-side slot reservation into an expert-major receive buffer, no regroup kernels (ops/csrc/ep.cu)
-        self.v2 = experts_per_rank > 0 and os.environ.get("MLXB200_EP_V2", "1") != "0"
         self.E_local = experts_per_rank
-        self.cap = max_tokens * top_k                      # rows one source can send to one destination
+        self.cap = max_tokens * top_k                      # pairs one rank routes per step (rows of its return buffer)
         W, cap, H = self.world, self.cap, hidden
+        rows = experts_per_rank * W * max_tokens
         self.off_recv_x = 0
-        if self.v2:
-            # [E_local][W * max_tokens][H] rows + their return addresses (u64) + [2][E_local] counters; arrival words live in the
-            # recv_count slot
-            rows = experts_per_rank * W * max_tokens
-            self.off_recv_meta = self.off_recv_x + rows * H * 2            # -> row_dst table
-            self.off_cnt = self.off_recv_meta + rows * 8
-            self.off_recv_count = (self.off_cnt + 2 * experts_per_rank * 4 + 255) // 256 * 256
-        else:
-            self.off_recv_meta = self.off_recv_x + W * cap * H * 2
-            self.off_recv_count = self.off_recv_meta + W * cap * 8
-        self.off_ret_y = (self.off_recv_count + W * 8 + 255) // 256 * 256     # recv_count: one u64 (count << 32 | step seq) per source
+        self.off_recv_meta = self.off_recv_x + rows * H * 2            # -> row_dst table
+        self.off_cnt = self.off_recv_meta + rows * 8
+        self.off_recv_count = (self.off_cnt + 2 * experts_per_rank * 4 + 255) // 256 * 256   # arrival words: one u64 per source
+        self.off_ret_y = (self.off_recv_count + W * 8 + 255) // 256 * 256
         self.off_flags = self.off_ret_y + cap * H * 4
         total = self.off_flags + 256
         self.base, handle = self.C.ipc_alloc(total)
@@ -68,20 +62,20 @@ class EPBuffers:
         # tables of peer addresses
         self.t_recv_x = [p + self.off_recv_x for p in self.peer]
         self.t_recv_meta = [p + self.off_recv_meta for p in self.peer]
+        self.t_cnt = [p + self.off_cnt for p in self.peer]
         self.t_recv_count = [p + self.off_recv_count for p in self.peer]
-        self.t_ret_y = [p + self.off_ret_y for p in self.peer]
         self.t_ret_flag = [p + self.off_flags + 128 for p in self.peer]
-        if self.v2:
-            self.t_cnt = [p + self.off_cnt for p in self.peer]
-            # my return buffer as mapped by every destination (the address a destination's down-projection epilogue stores to)
-            peers_all: List = [None] * W
-            dist.all_gather_object(peers_all, list(self.peer), group=group)
-            self.t_my_ret = [peers_all[d][self.rank] + self.off_ret_y for d in range(W)]
-            self.cnt = self.C.tensor_from_ptr(self.base + self.off_cnt, [2 * experts_per_rank], "int32", self.dev)
-            self._views = {}
-        # device-resident local state: [send_counts(world) | dispatch done ctr | down-GEMM tile ctr | regroup step seq seen |
-        #                               return arrivals expected | dispatch step seq | ... | error]
-        self.state = torch.zeros(W + 8, dtype=torch.int32, device="cuda")
+        # my return buffer as mapped by every destination (the address a destination's down-projection epilogue stores to)
+        peers_all: List = [None] * W
+        dist.all_gather_object(peers_all, list(self.peer), group=group)
+        self.t_my_ret = [peers_all[d][self.rank] + self.off_ret_y for d in range(W)]
+        self.cnt = self.C.tensor_from_ptr(self.base + self.off_cnt, [2 * experts_per_rank], "int32", self.dev)
+        self._views = {}
+        # device-resident local state, one int32 word each: dispatch CTAs done | down-GEMM tiles done | return arrivals the
+        # combine waits for | dispatch step sequence | error flag
+        self.state = torch.zeros(5, dtype=torch.int32, device="cuda")
+        self.done, self.tiles, self.ret_expected, self.seq = (self.state[j:j + 1] for j in range(4))
+        self.error_ptr = self.state[4:].data_ptr()
         self.ret_y = self.C.tensor_from_ptr(self.base + self.off_ret_y, [cap, H], "float32", self.dev)
         self.ret_flags_dev = torch.tensor(self.t_ret_flag, dtype=torch.int64, device="cuda")   # every source's return flag
         dist.barrier(group=group)
@@ -89,8 +83,13 @@ class EPBuffers:
     def error(self) -> bool:
         return bool(self.state[-1].item())
 
+    def stride(self, Tmax: int) -> int:
+        """Receive rows per expert for a step in which no rank routes more than ``Tmax`` tokens: ``world * Tmax`` rounded up to 64
+        (every rank computes the same value: ranks step in lock-step with equal batch shapes, or share a ``Tmax`` bound)."""
+        return min(self.world * self.max_tokens, (self.world * Tmax + 63) // 64 * 64)
+
     def recv_views(self, stride: int):
-        """(rows [E_local * stride, H] bf16, row_dst [E_local * stride] int64) over the v2 receive buffer for this step's stride."""
+        """(rows [E_local * stride, H] bf16, row_dst [E_local * stride] int64) over the receive buffer for this step's stride."""
         v = self._views.get(stride)
         if v is None:
             R = self.E_local * stride
@@ -100,7 +99,12 @@ class EPBuffers:
 
 
 class ExpertParallelMoE:
-    """One MoE layer's routed experts, sharded over the ranks of ``bufs``."""
+    """One MoE layer's routed experts, sharded over the ranks of ``bufs``.
+
+    A block is four launches: dispatch (slot reservation at the sender) -> grouped gate/up GEMM (acquires the arrivals itself) ->
+    grouped down GEMM (epilogue returns the rows) -> combine.  :meth:`forward` dispatches rows that were routed separately;
+    :meth:`route_forward` folds the pre-MoE RMSNorm and the router into the dispatch kernel and the next layer's input norm into
+    the combine."""
 
     def __init__(self, bufs: EPBuffers, Wg: LinearWeight, Wu: LinearWeight, Wd: LinearWeight, num_experts: int,
                  act: str = "silu", weights_are_local: bool = False):
@@ -115,114 +119,69 @@ class ExpertParallelMoE:
         pick = (lambda W: b200._dense(W)) if weights_are_local else (lambda W: b200._dense(W)[lo:hi].contiguous())
         self.wg, self.wu, self.wd = pick(Wg), pick(Wu), pick(Wd)
         self.act = b200.ACT_IDS[act]
+        self.peer_tokens_default = 0   # bound of the tokens any rank routes per step when ranks run different batch sizes
 
     def forward(self, x: torch.Tensor, idx: torch.Tensor, w: torch.Tensor, residual: Optional[torch.Tensor] = None,
                 out: Optional[torch.Tensor] = None, peer_tokens: Optional[int] = None, join=None) -> torch.Tensor:
         """``peer_tokens``: upper bound of the tokens *any* rank routes in this step (default: this rank's own ``T`` —
-        ranks stepping in lockstep with equal batch shapes); only sizes the temporaries of the local expert GEMMs."""
-        b, C = self.b, self.b.C
+        ranks stepping in lockstep with equal batch shapes); sizes the receive stride of the local expert GEMMs."""
+        b = self.b
         T, k = idx.shape
+
+        def dispatch(stride):
+            b.C.ep_dispatch_scatter(x, idx, self.E_local, b.rank, stride, b.t_recv_x, b.t_recv_meta, b.t_cnt, b.t_recv_count,
+                                    b.t_my_ret, b.seq, b.done, b.ret_expected)
+            return w, residual, join
+
+        return self._exchange(T, k, max(T, peer_tokens or self.peer_tokens_default), dispatch, out)
+
+    def route_forward(self, h, gate_w, route_kw: dict, pre_norm, residual_fn, out=None, next_norm=None):
+        """The whole block for ``1 <= T <= 1024``: the router with the pre-MoE RMSNorm and the dispatch folded in (``moe.cu``: the
+        token's CTA reserves its pairs' slots on the owners with remote atomics, stores the normalised row there and takes part in
+        the publication), then the experts and the combine with the next layer's input norm folded in.
+
+        ``h``: un-normalised residual stream; ``pre_norm = (weight, eps)``; ``residual_fn(normed)`` -> ``(residual, join)``: called
+        right after the router so the shared-expert branch (which consumes ``normed``) forks onto the side stream behind it;
+        ``next_norm = (weight, eps)`` or None.  Returns ``out`` or ``(out, normed_next)``."""
+        b, O = self.b, self.ops
+        T = h.shape[0]
+        k = int(route_kw["top_k"])
+        assert 1 <= T <= 1024, "the fused router + dispatch kernel takes 1 <= T <= 1024 tokens"
+        rk = route_kw
+        n_group, topk_group = O.route_groups(rk.get("method", "greedy"), rk.get("n_group", 1), rk.get("topk_group", 1))
+        normed = torch.empty_like(h)
+
+        def dispatch(stride):
+            idx, w = b.C.ep_route_dispatch(h, O._bf16(gate_w), k, n_group, topk_group, float(rk["scaling"]), bool(rk["norm_topk"]),
+                                           self.E_local, b.rank, stride, b.t_recv_x, b.t_recv_meta, b.t_cnt, b.t_recv_count,
+                                           b.t_my_ret, b.seq, b.done, b.ret_expected, O._bf16(pre_norm[0]), float(pre_norm[1]),
+                                           normed)
+            return (w, *residual_fn(normed))
+
+        return self._exchange(T, k, max(T, self.peer_tokens_default), dispatch, out, next_norm)
+
+    def _exchange(self, T, k, Tmax, dispatch, out, next_norm=None):
+        """``dispatch(stride)`` -> ``(w, residual, join)``, then the grouped GEMMs on the received rows and the combine."""
+        b, C, W = self.b, self.b.C, self.b.world
         assert T * k <= b.cap, "token batch exceeds the EP buffer capacity"
-        W = b.world
-        st = b.state
-        Tmax = max(T, peer_tokens or getattr(self, "peer_tokens_default", 0) or 0)
-        if b.v2:
-            return self._forward_v2(x, idx, w, residual, out, Tmax, join)
-        # 1) dispatch my pairs to the owners of their experts (remote stores + count/flag publication); also advances the
-        #    arrival target of this step's combine (st[W+3] += world)
-        C.ep_dispatch(x, idx, self.E_local, b.rank, b.cap, b.t_recv_x, b.t_recv_meta, b.t_recv_count, st[W + 4:W + 5],
-                      st[:W], st[W:W + 1], st[W + 3:W + 4])
-        # 2) wait for every source, bucket what I received by local expert; row_dst[r] = where row r's output must go
-        offs, total, x_perm, row_dst = C.ep_regroup(
-            b.base + b.off_recv_count, st[W + 2:W + 3].data_ptr(), st[-1:].data_ptr(),
-            b.base + b.off_recv_meta, b.base + b.off_recv_x, W, b.cap, self.E_local, b.H, b.dev, min(W * b.cap, W * Tmax * k), b.t_ret_y)
-        # 3) my experts: grouped swap-AB tcgen05 GEMMs on the received rows; the down-projection epilogue stores every output
-        #    row straight into its source rank's return buffer (peer memory) and the last tile bumps all sources' flags
-        max_rows = min(W * Tmax, x_perm.shape[0])  # upper bound of rows one expert can receive (every rank sends <= Tmax)
-        exp_rows = T * k  # balanced routing: a rank receives about as many pairs as it sends (only picks the token tile size)
-        h = C.grouped_linear(x_perm, self.wg, self.wu, offs, max_rows, self.act, False, None, None, None, exp_rows)
-        C.grouped_linear(h, self.wd, None, offs, max_rows, 0, True, row_dst, b.ret_flags_dev, st[W + 1:W + 2], exp_rows)
-        # 4) wait for all my pairs to come home + weighted combine (+ residual): one kernel
+        stride = b.stride(Tmax)
+        rows, row_dst = b.recv_views(stride)
+        w, residual, join = dispatch(stride)
+        max_rows = min(W * Tmax, stride)
+        arrive = (stride, b.base + b.off_recv_count, b.seq, b.error_ptr, W)
+        hmid = C.grouped_linear(rows, self.wg, self.wu, b.cnt, max_rows, self.act, False, None, None, None, T * k, *arrive, True)
+        C.grouped_linear(hmid, self.wd, None, b.cnt, max_rows, 0, True, row_dst, b.ret_flags_dev, b.tiles, T * k, *arrive, False)
         if join is not None:
             join.wait()  # ``residual`` (shared-expert branch) is produced on the side stream
-        return C.ep_combine(b.base + b.off_flags + 128, st[W + 3:W + 4], st[-1:].data_ptr(), b.ret_y, w, residual, out)
-
-
-    # (method of ExpertParallelMoE; placed after forward for readability)
-    pass
-
-
-def _forward_v2(self, x, idx, w, residual, out, Tmax, join):
-    """v2 exchange: 4 launches — dispatch (slot reservation at the sender) -> grouped gate/up GEMM (acquires the arrivals itself) ->
-    grouped down GEMM (epilogue returns the rows) -> combine.  The receive stride of this step is ``world * Tmax`` rows per expert
-    (every rank computes the same value: ranks step in lock-step with equal batch shapes, or pass ``peer_tokens``)."""
-    b, C = self.b, self.b.C
-    T, k = idx.shape
-    W, st = b.world, b.state
-    stride = min(W * b.max_tokens, (W * Tmax + 63) // 64 * 64)
-    rows, row_dst = b.recv_views(stride)
-    C.ep_dispatch_scatter(x, idx, self.E_local, b.rank, stride, b.t_recv_x, b.t_recv_meta, b.t_cnt, b.t_recv_count, b.t_my_ret,
-                          st[W + 4:W + 5], st[W:W + 1], st[W + 3:W + 4])
-    max_rows = min(W * Tmax, stride)
-    exp_rows = T * k
-    arrive, seq, err = b.base + b.off_recv_count, st[W + 4:W + 5], st[-1:].data_ptr()
-    h = C.grouped_linear(rows, self.wg, self.wu, b.cnt, max_rows, self.act, False, None, None, None, exp_rows, stride, arrive, seq, err, W, True)
-    C.grouped_linear(h, self.wd, None, b.cnt, max_rows, 0, True, row_dst, b.ret_flags_dev, st[W + 1:W + 2], exp_rows, stride, arrive, seq, err,
-                     W, False)
-    if join is not None:
-        join.wait()
-    return C.ep_combine(b.base + b.off_flags + 128, st[W + 3:W + 4], st[-1:].data_ptr(), b.ret_y, w, residual, out)
-
-
-ExpertParallelMoE._forward_v2 = _forward_v2
-
-
-def _route_forward(self, h, gate_w, route_kw: dict, pre_norm, residual_fn, out=None, next_norm=None):
-    """The whole expert-parallel block as FOUR kernels (v2 exchange, 1 <= T <= 1024): router with the pre-MoE RMSNorm and the
-    dispatch folded in (``moe.cu``: the token's CTA reserves its pairs' slots on the owners with remote atomics, stores the
-    normalised row there and takes part in the publication) -> grouped gate/up GEMM (acquires the arrivals) -> grouped down GEMM
-    (epilogue returns the rows) -> combine with the next layer's input norm folded in.
-
-    ``h``: un-normalised residual stream; ``pre_norm = (weight, eps)``; ``residual_fn(normed)`` -> ``(residual, join)``: called
-    right after the router so the shared-expert branch (which consumes ``normed``) forks onto the side stream behind it;
-    ``next_norm = (weight, eps)`` or None.  Returns ``out`` or ``(out, normed_next)``."""
-    b, C = self.b, self.b.C
-    from ..ops import b200 as O
-
-    T = h.shape[0]
-    k = int(route_kw["top_k"])
-    assert b.v2 and 1 <= T <= 1024 and T * k <= b.cap
-    W, st = b.world, b.state
-    Tmax = max(T, getattr(self, "peer_tokens_default", 0) or 0)
-    stride = min(W * b.max_tokens, (W * Tmax + 63) // 64 * 64)
-    rows, row_dst = b.recv_views(stride)
-    rk = dict(route_kw)
-    if rk.pop("method", "greedy") != "group_limited_greedy":
-        rk["n_group"], rk["topk_group"] = 1, 1
-    normed = torch.empty_like(h)
-    idx, w = C.ep_route_dispatch(h, O._bf16(gate_w), k, int(rk["n_group"]), int(rk["topk_group"]), float(rk["scaling"]),
-                                 bool(rk["norm_topk"]), self.E_local, b.rank, stride, b.t_recv_x, b.t_recv_meta, b.t_cnt,
-                                 b.t_recv_count, b.t_my_ret, st[W + 4:W + 5], st[W:W + 1], st[W + 3:W + 4],
-                                 O._bf16(pre_norm[0]), float(pre_norm[1]), normed)
-    residual, join = residual_fn(normed)
-    max_rows = min(W * Tmax, stride)
-    exp_rows = T * k
-    arrive, seq, err = b.base + b.off_recv_count, st[W + 4:W + 5], st[-1:].data_ptr()
-    hmid = C.grouped_linear(rows, self.wg, self.wu, b.cnt, max_rows, self.act, False, None, None, None, exp_rows, stride, arrive, seq, err, W, True)
-    C.grouped_linear(hmid, self.wd, None, b.cnt, max_rows, 0, True, row_dst, b.ret_flags_dev, st[W + 1:W + 2], exp_rows, stride, arrive, seq, err,
-                     W, False)
-    if join is not None:
-        join.wait()
-    flag, exp, errp = b.base + b.off_flags + 128, st[W + 3:W + 4], st[-1:].data_ptr()
-    if next_norm is not None and h.shape[1] <= 8192:
-        nxt = torch.empty_like(h)
-        res = C.ep_combine(flag, exp, errp, b.ret_y, w, residual, out, O._bf16(next_norm[0]), float(next_norm[1]), nxt)
-        return res, nxt
-    res = C.ep_combine(flag, exp, errp, b.ret_y, w, residual, out)
-    return res if next_norm is None else (res, O.rmsnorm(res, next_norm[0], next_norm[1]))
-
-
-ExpertParallelMoE.route_forward = _route_forward
+        combine = (b.base + b.off_flags + 128, b.ret_expected, b.error_ptr, b.ret_y, w, residual, out)
+        if next_norm is None:
+            return C.ep_combine(*combine)
+        H = b.H
+        if H <= 8192:   # (the fused combine-norm kernel holds a row of up to 8192)
+            nxt = torch.empty(T, H, dtype=torch.bfloat16, device=w.device)
+            return C.ep_combine(*combine, self.ops._bf16(next_norm[0]), float(next_norm[1]), nxt), nxt
+        res = C.ep_combine(*combine)
+        return res, self.ops.rmsnorm(res, next_norm[0], next_norm[1])
 
 
 class ExpertParallelMoERef:

@@ -1,7 +1,7 @@
 #!/bin/bash
 # A/B of environment toggles inside ONE gpurun call (same box, same clocks): each configuration runs the 1-GPU device-timed bench
 # twice, interleaved, so box-to-box variance (+-3 %) does not hide a 1-2 % effect.
-#   gpurun -- 'bash scripts/ab_bench.sh "MLXB200_FUSE_NORMS=1" "MLXB200_FUSE_NORMS=0" ...'
+#   bash scripts/ab_bench.sh "MLXB200_OVERLAP_SHARED=1" "MLXB200_OVERLAP_SHARED=0" ...
 mkdir -p gpurun_out
 for rep in 1 2; do
   for cfg in "$@"; do

@@ -24,10 +24,7 @@ if __name__ == "__main__":
     x = torch.randn(T, H, device="cuda", generator=g2).to(torch.bfloat16)
     res = torch.randn(T, H, device="cuda", generator=g2).to(torch.bfloat16)
     idx, w = b200.moe_route(x, gate, k)
-    # argv[1] == "v1": the regroup-kernel exchange; default: v2 (sender-side slot reservation, arrival wait fused into the GEMM)
-    v1 = len(sys.argv) > 1 and sys.argv[1] == "v1"
-    bufs = EPBuffers(H, 64, k) if v1 else EPBuffers(H, 64, k, experts_per_rank=E // world)
-    assert bufs.v2 == (not v1)
+    bufs = EPBuffers(H, 64, k, experts_per_rank=E // world)
     ep = ExpertParallelMoE(bufs, Wg, Wu, Wd, E)
     ok = True
     for it in range(3):  # several rounds: buffer reuse + counting flags
@@ -51,6 +48,6 @@ if __name__ == "__main__":
     if rank == 0:
         print(f"max err {err:.4g} graph {err_g:.4g}")
         if flag.item() == 1.0:
-            print("EP_OK", "v1" if v1 else "v2")
+            print("EP_OK")
     dist.barrier()
     dist.destroy_process_group()

@@ -1,7 +1,8 @@
 """torchrun worker: expert-parallel MoE under the conditions of a whole model — several layers sharing one ``EPBuffers`` called
 back to back with no host synchronisation in between, token counts that change from step to step (prefill chunk -> decode
 batch -> ...), two geometries (DeepSeek-V2-Lite's and the tiny test model's) — every output compared against the local MoE.
-``argv[1] == "v1"`` selects the regroup-kernel exchange.  Prints one line per (geometry, step) and EP_STRESS_OK on rank 0."""
+``argv[1]``: ``forward`` (rows routed separately, then ``ExpertParallelMoE.forward``) or ``fused`` (``route_forward``).  Prints
+one line per (geometry, step) and ``EP_STRESS_OK <mode>`` on rank 0."""
 import os
 import sys
 
@@ -54,13 +55,13 @@ def run_fused(H, I, E, k, Ts, layers, rank, world):
     return ok
 
 
-def run(H, I, E, k, Ts, layers, v1, rank, world):
+def run(H, I, E, k, Ts, layers, rank, world):
     g = torch.Generator(device="cuda").manual_seed(5)
     mk = lambda *s, sc=0.03: (torch.randn(*s, device="cuda", generator=g) * sc).to(torch.bfloat16)
     banks = [(LinearWeight(weight=mk(E, I, H)), LinearWeight(weight=mk(E, I, H)), LinearWeight(weight=mk(E, H, I)), mk(E, H, sc=0.05))
              for _ in range(layers)]
     maxT = max(Ts)
-    bufs = EPBuffers(H, maxT, k) if v1 else EPBuffers(H, maxT, k, experts_per_rank=E // world)
+    bufs = EPBuffers(H, maxT, k, experts_per_rank=E // world)
     eps = [ExpertParallelMoE(bufs, Wg, Wu, Wd, E) for Wg, Wu, Wd, _ in banks]
     g2 = torch.Generator(device="cuda").manual_seed(100 + rank)
     ok = True
@@ -107,7 +108,7 @@ def run(H, I, E, k, Ts, layers, v1, rank, world):
         ref = b200.moe_experts(x, idx, w, Wg, Wu, Wd, "silu")
         worst = max(worst, (got.float() - ref.float()).abs().max().item())
     ok = ok and worst < 2e-2 and not bufs.error()
-    print(f"[rank {rank}] H={H} E={E} graph T={T}: max err {worst:.4g}, {us:.1f} us per EP layer ({'v1' if v1 else 'v2'})", flush=True)
+    print(f"[rank {rank}] H={H} E={E} graph T={T}: max err {worst:.4g}, {us:.1f} us per EP layer", flush=True)
     return ok
 
 
@@ -116,22 +117,13 @@ if __name__ == "__main__":
     torch.cuda.set_device(lr)
     dist.init_process_group("nccl", device_id=torch.device("cuda", lr))
     rank, world = dist.get_rank(), dist.get_world_size()
-    v1 = len(sys.argv) > 1 and sys.argv[1] == "v1"
-    if len(sys.argv) > 1 and sys.argv[1] == "fused":
-        ok = run_fused(256, 128, 8, 3, [384, 16, 16, 48, 384, 16], 3, rank, world)
-        ok = run_fused(2048, 1408, 64, 6, [256, 64, 64, 48, 256, 64], 5, rank, world) and ok
-        flag = torch.tensor([1.0 if ok else 0.0], device="cuda")
-        dist.all_reduce(flag, op=dist.ReduceOp.MIN)
-        if rank == 0 and flag.item() == 1.0:
-            print("EP_STRESS_OK fused")
-        dist.barrier()
-        dist.destroy_process_group()
-        sys.exit(0)
-    ok = run(256, 128, 8, 3, [384, 16, 16, 48, 384, 16], 3, v1, rank, world)
-    ok = run(2048, 1408, 64, 6, [256, 64, 64, 48, 256, 64], 5, v1, rank, world) and ok
+    mode = sys.argv[1] if len(sys.argv) > 1 else "forward"
+    check = run_fused if mode == "fused" else run
+    ok = check(256, 128, 8, 3, [384, 16, 16, 48, 384, 16], 3, rank, world)
+    ok = check(2048, 1408, 64, 6, [256, 64, 64, 48, 256, 64], 5, rank, world) and ok
     flag = torch.tensor([1.0 if ok else 0.0], device="cuda")
     dist.all_reduce(flag, op=dist.ReduceOp.MIN)
     if rank == 0 and flag.item() == 1.0:
-        print("EP_STRESS_OK", "v1" if v1 else "v2")
+        print("EP_STRESS_OK", mode)
     dist.barrier()
     dist.destroy_process_group()

@@ -33,20 +33,22 @@ def test_serving_chain_parity(arch, transport, port):
     assert "SERVING_OK" in out, out[-3000:]
 
 
-@pytest.mark.parametrize("version,port", [("v2", 29574), ("v1", 29578)])
-def test_expert_parallel_moe(version, port):
-    """v2: sender-side slot reservation + arrival wait fused into the grouped GEMM; v1: regroup kernels on the receive side."""
-    out = _torchrun("ep_parity.py", [version], port=port)
-    assert "EP_OK " + version in out, out[-3000:]
+# (the "v2" test ids name the expert exchange as it was called when a second one still existed)
+@pytest.mark.parametrize("port", [pytest.param(29574, id="v2-29574")])
+def test_expert_parallel_moe(port):
+    """Sender-side slot reservation + arrival wait fused into the grouped GEMM == the local MoE, eagerly and under graph replay."""
+    out = _torchrun("ep_parity.py", [], port=port)
+    assert "EP_OK" in out, out[-3000:]
 
 
-@pytest.mark.parametrize("version,port", [("v2", 29584), ("v1", 29585), ("fused", 29586)])
-def test_expert_parallel_stress(version, port):
+@pytest.mark.parametrize("mode,port", [pytest.param("forward", 29584, id="v2-29584"), ("fused", 29586)])
+def test_expert_parallel_stress(mode, port):
     """Several EP layers sharing one buffer set, called back to back with no host synchronisation, token counts changing from step
-    to step (prefill chunk <-> decode batch), two geometries; every output must equal the local MoE bit for bit.  ``fused``: the
-    four-kernel block (norm + router + dispatch in one kernel, combine + next norm in one) against separate kernels."""
-    out = _torchrun("ep_stress.py", [version], port=port)
-    assert "EP_STRESS_OK " + version in out, out[-3000:]
+    to step (prefill chunk <-> decode batch), two geometries; every output must equal the local MoE bit for bit.  ``forward``: rows
+    routed separately; ``fused``: the four-kernel block (norm + router + dispatch in one kernel, combine + next norm in one)
+    against separate kernels."""
+    out = _torchrun("ep_stress.py", [mode], port=port)
+    assert "EP_STRESS_OK " + mode in out, out[-3000:]
 
 
 def test_expert_parallel_whole_model():
