@@ -39,6 +39,16 @@ void check_bf16(const Tensor& t, const char* name) {
 void check_rows(const Tensor& t, const char* name) {
   TORCH_CHECK(t.dim() == 2 && t.stride(1) == 1, name, " must be 2-D with a contiguous last dim");
 }
+// Operands the kernels read or write as 16-byte vectors (uint4 / float4) row by row: the first element of the view must be 16-byte
+// aligned and so must every row start.  The address comes from the storage, not data_ptr(), which is null for a tensor with no
+// rows, so a zero-row view is judged by where its rows would begin.  A single row never uses its row stride.
+void check_vec16(const Tensor& t, const char* name) {
+  const auto addr = reinterpret_cast<uintptr_t>(t.storage().data()) + static_cast<uintptr_t>(t.storage_offset() * t.element_size());
+  TORCH_CHECK(addr % 16 == 0, name, " must start on a 16-byte boundary (a column offset that is not a multiple of ",
+              16 / t.element_size(), " elements?)");
+  TORCH_CHECK(t.size(0) == 1 || t.stride(0) % (16 / t.element_size()) == 0, name, " row stride must be a multiple of ",
+              16 / t.element_size(), " elements (16 bytes)");
+}
 
 // ---- persistent scratch -----------------------------------------------------------------------------------------
 struct Scratch {
@@ -105,6 +115,8 @@ Tensor linear(const Tensor& x, const Tensor& w, const c10::optional<Tensor>& w2,
   TORCH_CHECK(w.size(1) == K, "x/w inner dims differ");
   Tensor out = out_.has_value() ? *out_ : torch::empty({T, N}, x.options().dtype(out_fp32 ? torch::kFloat32 : torch::kBFloat16));
   TORCH_CHECK(out.dim() == 2 && out.stride(1) == 1 && out.size(0) >= T && out.size(1) == N, "bad out tensor");
+  check_vec16(out, "out");
+  if (residual.has_value()) { check_bf16(*residual, "residual"); check_rows(*residual, "residual"); check_vec16(*residual, "residual"); }
   if (T == 0) return out;
   b200::GemmArgs a;
   a.x = x.data_ptr(); a.x_rows = T; a.ld_x = x.stride(0);
@@ -112,7 +124,7 @@ Tensor linear(const Tensor& x, const Tensor& w, const c10::optional<Tensor>& w2,
   if (w2.has_value()) { check_bf16(*w2, "w2"); TORCH_CHECK(w2->sizes() == w.sizes() && w2->stride(0) == w.stride(0)); a.w2 = w2->data_ptr(); }
   a.m = (int)T; a.n = (int)N; a.k = (int)K; a.max_rows = (int)T;
   a.out = out.data_ptr(); a.ld_out = out.stride(0); a.out_fp32 = out.scalar_type() == torch::kFloat32;
-  if (residual.has_value()) { check_bf16(*residual, "residual"); check_rows(*residual, "residual"); a.residual = residual->data_ptr(); a.ld_res = residual->stride(0); }
+  if (residual.has_value()) { a.residual = residual->data_ptr(); a.ld_res = residual->stride(0); }
   if (bias.has_value()) { check_bf16(*bias, "bias"); a.bias = bias->data_ptr(); }
   a.act = (int)act; a.softcap = (float)softcap;
   int sp = splits > 0 ? (int)splits : auto_splits((int)T, (int)N, (int)K, false);
@@ -200,6 +212,8 @@ Tensor linear_q(const Tensor& x, const Tensor& wq, const Tensor& scales_t, const
   check_q(wq, scales_t, biases_t, N, K, bits, group);
   Tensor out = out_.has_value() ? *out_ : torch::empty({T, N}, x.options().dtype(out_fp32 ? torch::kFloat32 : torch::kBFloat16));
   TORCH_CHECK(out.dim() == 2 && out.stride(1) == 1 && out.size(0) >= T && out.size(1) == N, "bad out tensor");
+  check_vec16(out, "out");
+  if (residual.has_value()) { check_bf16(*residual, "residual"); check_rows(*residual, "residual"); check_vec16(*residual, "residual"); }
   if (T == 0) return out;
   b200::GemmArgs a;
   a.x = x.data_ptr(); a.x_rows = T; a.ld_x = x.stride(0);
@@ -211,7 +225,7 @@ Tensor linear_q(const Tensor& x, const Tensor& wq, const Tensor& scales_t, const
   }
   a.m = (int)T; a.n = (int)N; a.k = (int)K; a.max_rows = (int)T;
   a.out = out.data_ptr(); a.ld_out = out.stride(0); a.out_fp32 = out.scalar_type() == torch::kFloat32;
-  if (residual.has_value()) { check_bf16(*residual, "residual"); check_rows(*residual, "residual"); a.residual = residual->data_ptr(); a.ld_res = residual->stride(0); }
+  if (residual.has_value()) { a.residual = residual->data_ptr(); a.ld_res = residual->stride(0); }
   if (bias.has_value()) { check_bf16(*bias, "bias"); a.bias = bias->data_ptr(); }
   a.act = (int)act; a.softcap = (float)softcap;
   // quantised weights: 3.5x fewer bytes per tile, so batches of >= 64 tokens use the persistent kernel un-split; tiny decode
@@ -272,10 +286,14 @@ Tensor rmsnorm(const Tensor& x, const Tensor& w, double eps, bool gemma, const c
   const c10::cuda::CUDAGuard guard(x.device());
   Tensor out = out_.has_value() ? *out_ : torch::empty({x.size(0), x.size(1)}, x.options());
   TORCH_CHECK(out.scalar_type() == torch::kBFloat16 && out.stride(1) == 1 && out.size(0) >= x.size(0) && out.size(1) == x.size(1), "bad out tensor");
+  check_vec16(x, "x"); check_vec16(out, "out");
   unsigned int* done = nullptr;
   if (signal_flag_ptr != 0) done = reinterpret_cast<unsigned int*>(scratch().get_counters(x.device()).data_ptr<int>()) + 65532;
   const void* res = nullptr; long long ldr = 0;
-  if (residual.has_value()) { check_bf16(*residual, "residual"); check_rows(*residual, "residual"); res = residual->data_ptr(); ldr = residual->stride(0); }
+  if (residual.has_value()) {
+    check_bf16(*residual, "residual"); check_rows(*residual, "residual"); check_vec16(*residual, "residual");
+    res = residual->data_ptr(); ldr = residual->stride(0);
+  }
   LAUNCH_OK(b200::rmsnorm_launch(x.data_ptr(), x.stride(0), w.data_ptr(), res, ldr, out.data_ptr(), out.stride(0), (int)x.size(0),
                                (int)x.size(1), (float)eps, gemma, cur_stream(), reinterpret_cast<uint32_t*>(signal_flag_ptr),
                                (uint32_t)signal_value, done));
